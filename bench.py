@@ -70,7 +70,22 @@ def parse():
                          "workload it discards every visit (DESIGN.md 9b)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (solved Jones, return code, mean nu, "
+                         "initial and final residual) as DIR/<workload>_<name>.npy, float64, so two "
+                         "builds can be compared output for output on the same seeded inputs (the "
+                         "reference arm: DIR/reference_<workload>_<name>.npy)")
     return ap.parse_args()
+
+
+def dump_outputs(args, name, arrays):
+    """rank 0 only: the arrays a caller of the timed path receives, one .npy per array"""
+    if not args.dump_outputs:
+        return
+    os.makedirs(args.dump_outputs, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(args.dump_outputs, "%s_%s.npy" % (name, k)),
+                np.asarray(a, dtype=np.float64))
 
 
 def solve_args(name):
@@ -204,9 +219,10 @@ def ncu_traffic(workload="C2"):
 # ---------------------------------------------------------------------------------------------
 # reference (CPU) arm — the only place besides tests/ and smoke() that may execute oracle/
 # ---------------------------------------------------------------------------------------------
-def cpu_reference_run(steps, warmup, seed):
+def cpu_reference_run(steps, warmup, seed, outputs=None):
     """times the reference's own sagefit_visibilities (oracle/_ref) on a bounded sample of the
-    workload with every host thread; returns (units/s, seconds per step, description)"""
+    workload with every host thread; returns (units/s, seconds per step, description).  `outputs`,
+    if given, receives what the last step returned (solved Jones and result values)."""
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import refdirac
     from sagecal_b200 import synth
@@ -231,11 +247,13 @@ def cpu_reference_run(steps, warmup, seed):
         x = pr.x.copy()
         pp = pr.pp0.copy()
         t0 = time.perf_counter()
-        ref.sagefit_visibilities(pr.u, pr.v, pr.w, x, pr.N, pr.Nbase, pr.tilesz, barr, sky, pr.coh,
-                                 pp, Nt=cores, **SOLVE)
+        res = ref.sagefit_visibilities(pr.u, pr.v, pr.w, x, pr.N, pr.Nbase, pr.tilesz, barr, sky,
+                                       pr.coh, pp, Nt=cores, **SOLVE)
         t1 = time.perf_counter()
         if it >= warmup:
             ts.append(t1 - t0)
+    if outputs is not None:
+        outputs.update(jones=pp, result=res)
     sec = float(np.mean(ts))
     desc = ("reference sagefit_visibilities (oracle/_ref, gcc -O2, OpenBLAS %d threads, Nt=%d) on "
             "N=%d M=%d tilesz=%d, %d steps" % (cores, cores, pr.N, pr.M, pr.tilesz, steps))
@@ -321,13 +339,14 @@ def run_reference_arm(args):
     if rank != 0:
         return
     shape = workload_shape(args.workload)
-    steps = max(1, min(args.steps, 3))
-    warm = 1 if args.warmup > 0 else 0
-    v, sec, desc = cpu_reference_run(steps, warm, shape["seed"])
+    steps, warm = args.steps, args.warmup
+    outputs = {}
+    v, sec, desc = cpu_reference_run(steps, warm, shape["seed"], outputs)
     cores = min(os.cpu_count() or 1, 32)
     if v is None:
         emit({"impl": "reference", "unavailable": desc})
         return
+    dump_outputs(args, "reference_" + args.workload, outputs)
     line = {
         "impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus,
         "steps": steps, "warmup": warm, "ms_per_step": sec * 1e3, "higher_is_better": True,
@@ -496,6 +515,8 @@ def run_workload(name, args, ctx, with_cpu=True):
             res = dp.sagefit(pp, None, **SOLVE_W)
         e1.record(stream)
         torch.cuda.synchronize()
+        if rank == 0:
+            dump_outputs(args, name, {"jones": pp, "result": res})
         if world > 1:
             dist.barrier()
         clk = clocks.stop()
@@ -736,6 +757,8 @@ def run_consensus(args, ctx):
             sb, pp, hist = solve(dp)
         e1.record(stream)
         torch.cuda.synchronize()
+        if rank == 0:
+            dump_outputs(args, "C5", {"jones": pp, "history": hist})
         if world > 1:
             dist.barrier()
         clk = clocks.stop()

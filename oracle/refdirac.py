@@ -103,6 +103,17 @@ class RefDirac(DiracAPI):
         self.lib.ref_mylm_jac_single_pth(dptr(pblk), dptr(jac), m, n, md)
         return jac.reshape(n, m)
 
+    def normal_eq(self, pblk, xs, md, wt=None):
+        """(e.e, J^T e, J^T J) of one (cluster, chunk) from the dense Jacobian and the model, with
+        J <- wt.J and e <- wt.e when weights are given (robustlm.c:2298-2316)"""
+        n = len(xs)
+        J = self.lm_jac(pblk, md, n)
+        e = xs - self.lm_func(pblk, md, n)
+        if wt is not None:
+            J = J * wt[:, None]
+            e = wt * e
+        return e @ e, J.T @ e, J.T @ J
+
     def cost(self, pp, x, md, robust=False):
         f = self.lib.ref_robust_cost_func if robust else self.lib.ref_cost_func
         return f(dptr(pp), len(pp), dptr(x), len(x), md)

@@ -12,24 +12,31 @@ def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
 
 
+def _golden_ref(request, tag, path, load):
+    """the compiled reference where it is built, else its recorded answers (tests/refgolden.py)"""
+    import refgolden
+    m = refgolden.mode(os.path.exists(path))
+    if m == "live":
+        return load()
+    if m == "record":
+        request.addfinalizer(refgolden.save)
+        return refgolden.GoldenRef(tag, load())
+    return refgolden.GoldenRef(tag)
+
+
 @pytest.fixture(scope="session")
-def ref():
+def ref(request):
     """compiled reference CPU path (oracle/_ref), test infrastructure only"""
     import refdirac
-    if not refdirac.available():
-        pytest.skip("oracle/_ref/libdirac_ref.so not built (make -C oracle)")
-    return refdirac.load()
+    return _golden_ref(request, "ref", refdirac.REF_PATH, refdirac.load)
 
 
 @pytest.fixture(scope="session")
-def refser():
+def refser(request):
     """the compiled reference with the worker threads of its robust RTR / NSD solvers run
     synchronously (oracle/ref_shim_rtr_serial.c): deterministic pin of solver_mode 5 and 6"""
     import refdirac
-    import os
-    if not os.path.exists(refdirac.SERIAL_PATH):
-        pytest.skip("oracle/_ref/libdirac_ref_serial.so not built (make -C oracle)")
-    return refdirac.load_serial()
+    return _golden_ref(request, "refser", refdirac.SERIAL_PATH, refdirac.load_serial)
 
 
 @pytest.fixture(scope="session")

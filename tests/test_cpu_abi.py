@@ -1,5 +1,6 @@
 """CPU: the C-ABI library loads and exports every symbol include/dirac_b200.h declares; host-only
 helpers (index / flag work) are bit-exact against the reference.  No compute calls."""
+import json
 import os
 import re
 
@@ -8,8 +9,10 @@ import pytest
 
 from sagecal_b200 import lib as blib
 from sagecal_b200.dirac_api import barr_to_numpy
+from util import known
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+REF_SIGNATURES = os.path.join(ROOT, "tests", "golden", "ref_signatures.json")
 
 
 @pytest.fixture(scope="module")
@@ -53,7 +56,9 @@ def test_preset_flags_bit_exact(product, ref):
         x = xs.copy()
         lib.preset_flags_and_data(flag.copy(), barr, x)
         res.append((barr_to_numpy(barr, n)[2], x))
-    assert np.array_equal(res[0][0], res[1][0]) and np.array_equal(res[0][1], res[1][1])
+    k = known(res[0][1])
+    assert np.array_equal(res[0][0], res[1][0])
+    assert np.array_equal(res[0][1][k], res[1][1][k])
 
 
 def test_whiten_data_bit_exact(product, ref):
@@ -69,7 +74,8 @@ def test_whiten_data_bit_exact(product, ref):
             x = xs.copy()
             lib.whiten_data(x, u, v, 150e6, Nt)
             out.append(x)
-        assert np.array_equal(out[0], out[1])
+        k = known(out[0])
+        assert np.array_equal(out[0][k], out[1][k])
         d = np.hypot(u, v) * 150e6
         assert (d > 400).any() and (d < 400).any()
         untouched = np.repeat(d > 400, 8)
@@ -122,17 +128,33 @@ def _c_declarations(path):
     return out
 
 
-def test_signatures_equal_the_reference_headers():
-    """every reference-named entry point is declared with the reference's own parameter type list
-    (complex double * spelled double *); the *_hbb pair carries the HAVE_CUDA variant of its name"""
-    refroot = "/root/reference/src/lib"
-    if not os.path.isdir(refroot):
-        pytest.skip("reference headers not present on this box")
-    ours = _c_declarations(os.path.join(ROOT, "include", "dirac_b200.h"))
+def _reference_declarations(names):
+    """{entry point: [parameter type lists]} of the reference's Dirac.h, Dirac_common.h and
+    Dirac_radio.h for the given names: parsed where the reference sources are (DIRAC_REFERENCE),
+    else read back from tests/golden/ref_signatures.json (stored by a run with
+    DIRAC_REF_GOLDEN=record)"""
+    if not os.environ.get("DIRAC_REFERENCE"):
+        with open(REF_SIGNATURES) as f:
+            return json.load(f)
+    refroot = os.path.join(os.environ["DIRAC_REFERENCE"], "src", "lib")
     ref = {}
     for h in ("Dirac/Dirac.h", "Dirac/Dirac_common.h", "Radio/Dirac_radio.h"):
         for k, v in _c_declarations(os.path.join(refroot, h)).items():
             ref.setdefault(k, []).extend(v)
+    ref = {k: v for k, v in ref.items() if k in names}
+    if os.environ.get("DIRAC_REF_GOLDEN") == "record":
+        with open(REF_SIGNATURES, "w") as f:
+            json.dump(ref, f, indent=1, sort_keys=True)
+            f.write("\n")
+    return ref
+
+
+def test_signatures_equal_the_reference_headers():
+    """every reference-named entry point is declared with the reference's own parameter type list
+    (complex double * spelled double *); the *_hbb pair carries the HAVE_CUDA variant of its name"""
+    ours = _c_declarations(os.path.join(ROOT, "include", "dirac_b200.h"))
+    bases = {n[:-4] if n.endswith("_hbb") else n for n in ours if not n.startswith("dirac_b200")}
+    ref = _reference_declarations(bases)
     checked = 0
     for name, sigs in ours.items():
         if name.startswith("dirac_b200"):
@@ -184,4 +206,5 @@ def test_extract_phases_matches_reference(ref):
         want, got = np.zeros(8 * N), np.zeros(8 * N)
         ref.lib.extract_phases(dptr(p.copy()), dptr(want), N, 10)
         L.dirac_b200_extract_phases(dptr(p), dptr(got), N, 10)
-        assert np.max(np.abs(got - want)) < 1e-10, np.max(np.abs(got - want))
+        k = known(want)
+        assert np.max(np.abs(got - want)[k]) < 1e-10, np.max(np.abs(got - want)[k])

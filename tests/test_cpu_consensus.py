@@ -16,6 +16,11 @@ from sagecal_b200 import consensus as cons
 from sagecal_b200.dirac_api import dptr
 
 
+def vptr(a):
+    """a void * to the array that keeps the array with it (numpy's data_as)"""
+    return a.ctypes.data_as(C.c_void_p)
+
+
 @pytest.fixture(scope="module")
 def capi():
     from sagecal_b200 import lib
@@ -29,7 +34,7 @@ def test_basis_matches_reference(capi, ref, ptype):
         B = cons.basis(capi, freqs, 150e6, Npoly, ptype)
         Br = np.zeros((8, Npoly))
         ref.lib.setup_polynomials.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_double, C.c_int]
-        ref.lib.setup_polynomials(Br.ctypes.data, Npoly, 8, freqs.ctypes.data, 150e6, ptype)
+        ref.lib.setup_polynomials(vptr(Br), Npoly, 8, vptr(freqs), 150e6, ptype)
         assert np.allclose(B, Br, rtol=1e-14, atol=1e-300)
 
 
@@ -45,7 +50,7 @@ def test_prod_inverse_matches_reference(capi, ref):
         ref.lib.find_prod_inverse_full.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                                    C.c_void_p, C.c_int]
         Bc = np.ascontiguousarray(B)
-        ref.lib.find_prod_inverse_full(Bc.ctypes.data, Bir.ctypes.data, Npoly, 8, M, rho.ctypes.data, 2)
+        ref.lib.find_prod_inverse_full(vptr(Bc), vptr(Bir), Npoly, 8, M, vptr(rho), 2)
         assert np.max(np.abs(Bi - Bir)) <= 1e-9 * np.max(np.abs(Bir))
 
 

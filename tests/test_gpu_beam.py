@@ -9,7 +9,7 @@ import ctypes as C
 import numpy as np
 import pytest
 
-from util import small_problem, relerr, perturbed_jones
+from util import small_problem, relerr, perturbed_jones, known
 from sagecal_b200.dirac_api import BeamSetup, SkyModel, elementcoeff, dptr
 
 pytestmark = pytest.mark.gpu
@@ -70,12 +70,13 @@ def test_coherencies_withbeam(api, ref, mode, tile):
     got = api.precalculate_coherencies_withbeam(pr.u, pr.v, pr.w, pr.N, pr.Nbase1, b.fresh_barr(),
                                                 sky, pr.freq0, pr.fdelta, beam, uvmin=30.0,
                                                 uvmax=1e5)
-    assert np.max(np.abs(want)) > 0
+    assert np.max(np.abs(want[known(want)])) > 0
     assert relerr(got, want) < 1e-10, relerr(got, want)
     # the beam matters: the result differs from the beam-less coherencies
     plain = ref.precalculate_coherencies(pr.u, pr.v, pr.w, pr.N, pr.Nbase1, b.fresh_barr(), sky,
                                          pr.freq0, pr.fdelta, uvmin=30.0, uvmax=1e5)
-    assert relerr(want, plain) > 1e-3
+    k = known(want) & known(plain)
+    assert relerr(want[k], plain[k]) > 1e-3
 
 
 @pytest.mark.parametrize("mode,tile", [("full", False), ("full_wb", True), ("array", True)],
@@ -94,7 +95,7 @@ def test_predict_and_residual_withbeam(api, ref, mode, tile):
     # full-resolution residual with solutions and the correction by cluster 1
     pp = perturbed_jones(pr, seed=4, amp=0.1)
     rng = np.random.default_rng(2)
-    x0 = xa + rng.normal(0, 0.01, xa.shape)
+    x0 = xb + rng.normal(0, 0.01, xb.shape)   # (xa may be a stored sample of the reference's)
     ra, rb = x0.copy(), x0.copy()
     ref.calculate_residuals_multifreq_withbeam(pr.u, pr.v, pr.w, pp, ra, pr.N, pr.Nbase, pr.tilesz,
                                                b.barr, sky, freqs, pr.fdelta * 2, beam, ccid=1)

@@ -4,7 +4,7 @@ order only."""
 import numpy as np
 import pytest
 
-from util import small_problem, perturbed_jones, relerr
+from util import small_problem, perturbed_jones, relerr, known
 from sagecal_b200 import lib as blib
 
 pytestmark = pytest.mark.gpu
@@ -33,7 +33,7 @@ def test_predict_full(api, ref, bound):
         c, res = dp.predict(pp, out_mode=1, cost_mode=1)
     assert relerr(got, want) < 1e-13
     assert relerr(res, pr.x - want) < 1e-13
-    assert abs(c - np.sum((pr.x - want) ** 2)) <= 1e-12 * c
+    assert abs(c - ref.cost(pp, pr.x, md)) <= 1e-12 * c
     # flagged rows carry no model (lmfit.c:78-81)
     assert np.all(got.reshape(-1, 8)[pr.flag != 0] == 0.0)
 
@@ -76,12 +76,11 @@ def test_normal_equations(api, ref, bound):
                                  tileoff=t0)
                 nn = 8 * (t1 - t0) * pr.Nbase
                 xs = xd[8 * t0 * pr.Nbase: 8 * t1 * pr.Nbase]
-                J = ref.lm_jac(pblk, md, nn)
-                e = xs - ref.lm_func(pblk, md, nn)
+                ee, JTe_ref, JTJ_ref = ref.normal_eq(pblk, xs, md)
                 c, JTJ, JTe = dp.normal_eq(k, ck, pblk, xd)
-                assert abs(c - e @ e) <= 1e-12 * (e @ e)
-                assert relerr(JTe, J.T @ e) < 1e-11
-                assert relerr(JTJ, J.T @ J) < 1e-11
+                assert abs(c - ee) <= 1e-12 * ee
+                assert relerr(JTe, JTe_ref) < 1e-11
+                assert relerr(JTJ, JTJ_ref) < 1e-11
                 assert np.array_equal(JTJ, JTJ.T)
 
 
@@ -107,12 +106,11 @@ def test_weighted_normal_equations(api, ref, bound):
                                  tileoff=t0)
                 nn = 8 * (t1 - t0) * pr.Nbase
                 sl = slice(8 * t0 * pr.Nbase, 8 * t1 * pr.Nbase)
-                J = ref.lm_jac(pblk, md, nn) * wt[sl][:, None]
-                e = wt[sl] * (pr.x[sl] - ref.lm_func(pblk, md, nn))
+                ee, JTe_ref, JTJ_ref = ref.normal_eq(pblk, pr.x[sl], md, wt[sl])
                 c, JTJ, JTe = dp.normal_eq_weighted(k, ck, pblk, pr.x, wt)
-                assert abs(c - e @ e) <= 1e-12 * (e @ e)
-                assert relerr(JTe, J.T @ e) < 1e-11
-                assert relerr(JTJ, J.T @ J) < 1e-11
+                assert abs(c - ee) <= 1e-12 * ee
+                assert relerr(JTe, JTe_ref) < 1e-11
+                assert relerr(JTJ, JTJ_ref) < 1e-11
                 assert relerr(JTJ, JTJ.T) < 1e-13
 
 
@@ -250,4 +248,5 @@ def test_calculate_residuals_multifreq(api, ref, ccid, nchunk, phase_only):
     # (phase_only: the correction goes through a joint diagonalisation by Jacobi rotations,
     # manifold_average.c:399-610, restated on the host with its own 3x3 eigen-solver)
     assert relerr(xb, xa) < (1e-9 if phase_only else 1e-11)
-    assert relerr(xa, x0) > 1e-3   # something was subtracted
+    k = known(xa)
+    assert relerr(xa[k], x0[k]) > 1e-3   # something was subtracted
